@@ -27,12 +27,16 @@ collective on the data path (hash partitions are independent, SURVEY.md §8e).
              sizes 8..256 MB, bottommost forced, roofline fraction per size.
   ycsb_a   = BASELINE.json configs[4] at small scale (N=1): 50/50 put+get through the rrdb surface.
 
-Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned (see dump_compaction, dump_reads) as
+DIR/<name>.npy, so that two builds can be compared output for output; the inputs are seeded and identical from run to run.
+
+Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
 import argparse
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -43,6 +47,7 @@ from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -126,11 +131,96 @@ def cpu_block_runs(runs):
 
 
 def cpu_compaction(bruns, threads: int):
-    """oracle block-level compaction on host cores; returns (merged GB/s, seconds, stats)."""
+    """oracle block-level compaction on host cores; returns (merged GB/s, seconds, stats, merged block run)."""
     import oracle_py as orc
     fp = orc.filter_params(enabled=True)
-    _out, st, secs = orc.compact_blocks(bruns, True, fp, NOW, threads)
-    return st.in_bytes / secs / 1e9, secs, st
+    out, st, secs = orc.compact_blocks(bruns, True, fp, NOW, threads)
+    return st.in_bytes / secs / 1e9, secs, st, out
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# --dump-outputs: float32 / float64 arrays, under 50 MB in all whatever the read batch sizes
+# ---------------------------------------------------------------------------------------------------------------------
+DUMP_RECORDS = 16384     # merged records sampled: 16384 x (50 B key + 268 B value) bytes as float32 is ~21 MB
+DUMP_REQUESTS = 1 << 20  # per-request arrays of the read legs (every request at the default batch sizes)
+
+
+def sample_index(n: int, cap: int, seed: int) -> np.ndarray:
+    """0..n-1, or a fixed seeded sorted sample of cap of them"""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, size=cap, replace=False))
+
+
+def padded_rows(buf: np.ndarray, off: np.ndarray, pick: np.ndarray) -> np.ndarray:
+    """buf[off[i]:off[i + 1]] for i in pick as float32 rows, zero-padded to the longest (the lengths are dumped beside)"""
+    start, length = off[pick].astype(np.int64), (off[pick + 1] - off[pick]).astype(np.int64)
+    col = np.arange(int(length.max(initial=0)))
+    inside = col < length[:, None]
+    return np.where(inside, buf[np.where(inside, start[:, None] + col, 0)], 0).astype(np.float32)
+
+
+def gather(buf: np.ndarray, start: np.ndarray, length: np.ndarray) -> np.ndarray:
+    """buf[start[i]:start[i] + length[i]] for every i, concatenated"""
+    start, length = start.astype(np.int64), length.astype(np.int64)
+    end = np.cumsum(length)
+    total = int(end[-1]) if end.size else 0
+    return buf[np.repeat(start - end + length, length) + np.arange(total)]
+
+
+def digest(*arrays) -> np.ndarray:
+    """SHA-256 of the arrays' bytes, as 32 float32 values 0..255: equal iff the whole output is (not just the sample)"""
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).view(np.uint8))
+    return np.frombuffer(h.digest(), np.uint8).astype(np.float32)
+
+
+def write_arrays(out_dir: str, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_compaction(out_dir: str, stats, merged) -> None:
+    """the compaction step's statistics (STAT_FIELDS, as the oracle reports them too), a seeded sample of the merged
+    records (key and value bytes, lengths, sequence numbers, types) and a digest of the whole merged run"""
+    pick = sample_index(merged.n, DUMP_RECORDS, seed=0)
+    write_arrays(out_dir, {
+        "compaction_stats": np.array([int(getattr(stats, f)) for f in STAT_FIELDS], np.float64),
+        "compaction_sample_index": pick.astype(np.float64),
+        "compaction_sample_keys": padded_rows(merged.keys, merged.key_off, pick),
+        "compaction_sample_key_len": (merged.key_off[pick + 1] - merged.key_off[pick]).astype(np.float32),
+        "compaction_sample_values": padded_rows(merged.vals, merged.val_off, pick),
+        "compaction_sample_value_len": (merged.val_off[pick + 1] - merged.val_off[pick]).astype(np.float32),
+        "compaction_sample_seq": merged.seq[pick].astype(np.float64),
+        "compaction_sample_type": merged.type[pick].astype(np.float32),
+        "compaction_digest": digest(merged.keys, merged.key_off, merged.vals, merged.val_off, merged.seq, merged.type),
+    })
+
+
+def dump_reads(out_dir: str, gres, garena: np.ndarray, sb) -> None:
+    """the last get batch (status, expire_ts, expired flag, value length per key; digest of the values found) and the last
+    prefix-scan batch (status and record count per request; digest of the records returned)"""
+    g = np.ctypeslib.as_array(gres)
+    found = g["status"] == 0
+    gi = sample_index(g.shape[0], DUMP_REQUESTS, seed=1)
+    s = np.ctypeslib.as_array(sb.results)
+    si = sample_index(s.shape[0], DUMP_REQUESTS, seed=2)
+    n_kv = int(sb.kbase[-1])
+    kv = sb.kvs.reshape(-1, 5)[:n_kv]
+    base = np.repeat(sb.abase[:-1], np.diff(sb.kbase)).astype(np.int64)
+    write_arrays(out_dir, {
+        "get_status": g["status"][gi].astype(np.float32),
+        "get_expire_ts": g["expire_ts"][gi].astype(np.float64),
+        "get_expired": g["expired"][gi].astype(np.float32),
+        "get_value_len": g["value_len"][gi].astype(np.float32),
+        "get_values_digest": digest(found, g["value_len"][found], gather(garena, g["value_off"][found], g["value_len"][found])),
+        "scan_status": s["status"][si].astype(np.float32),
+        "scan_n_kvs": s["n_kvs"][si].astype(np.float32),
+        "scan_records_digest": digest(np.diff(sb.kbase), kv[:, [1, 3]], gather(sb.arena, base + kv[:, 0], kv[:, 1]),
+                                      gather(sb.arena, base + kv[:, 2], kv[:, 3])),
+    })
 
 
 def zipf_ids(rng, n_items: int, n: int, theta: float = 0.99):
@@ -166,9 +256,12 @@ def reference_arm(args, rank: int, world: int):
     n = args.records_per_run
     bruns = cpu_block_runs(gen_runs(n, 1000))
     vals = []
-    for _ in range(args.warmup + args.steps):
-        gbs, secs, st = cpu_compaction(bruns, threads)
+    for i in range(args.warmup + args.steps):
+        gbs, secs, st, out = cpu_compaction(bruns, threads)
         vals.append((gbs, secs))
+        if args.dump_outputs and i == args.warmup + args.steps - 1:
+            dump_compaction(args.dump_outputs, st, out.decode().records())
+        del out
     in_bytes = int(st.in_bytes)
     timed = vals[args.warmup:]
     ms = 1e3 * sum(s for _, s in timed) / len(timed)
@@ -273,9 +366,8 @@ def sharded_read_leg(pgs, torch, dist, eng, rank, world, args, barrier, check_cp
     list(pool.map(serve, work))  # warm-up pass (also the answer that is checked below)
     first = dict(tot)
     verify[0] = False
-    reps = max(3, args.steps)
     walls = []
-    for _ in range(reps):
+    for _ in range(args.steps):
         tot.update(found=0, returned=0, kernel_ms=0.0, calls=0)
         barrier()
         w0 = time.perf_counter()
@@ -370,7 +462,7 @@ def sweep_leg(pgs, eng, args, peak):
         part = eng.partition(app_id=3, pidx=mb)
         ids = part.upload_many([pgs.build_run(r) for r in runs], levels=[4, 3, 2, 1, 0])
         ms = []
-        for i in range(2 + 3):
+        for i in range(2 + args.steps):
             res = part.compact(ids, out_level=4, bottommost=1, now=NOW, enabled=True, flags=3)
             if i >= 2:
                 ms.append(res.merge_kernel_ms)
@@ -382,7 +474,7 @@ def sweep_leg(pgs, eng, args, peak):
                     "roofline_frac": algo / (k_ms / 1e3) / 1e9 / peak})
         part.close()
     return {"workload": "manual_compact sweep: 5 runs (L0..L4) of equal size, 30 % of the values expired, TTL filter on, bottommost forced "
-                        "(BASELINE.json configs[3]); merge kernels timed with CUDA events, mean of 3 after 2 warm-ups",
+                        f"(BASELINE.json configs[3]); merge kernels timed with CUDA events, mean of {args.steps} after 2 warm-ups",
             "sizes": out}
 
 
@@ -438,7 +530,11 @@ def main():
     ap.add_argument("--sweep-mb", type=int, nargs="*", default=[8, 16, 32, 64, 128, 256])
     ap.add_argument("--ycsb-keys", type=int, default=20000)
     ap.add_argument("--ycsb-ops", type=int, default=20000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -490,8 +586,8 @@ def main():
     stream = torch.cuda.ExternalStream(eng.stream, device=torch.device("cuda", local_rank))
     KEEP = 1 | 2  # PGS_COMPACT_KEEP_INPUTS | PGS_COMPACT_DISCARD_OUTPUT: repeat the same job
 
-    def step():
-        return part.compact(ids, out_level=1, bottommost=1, now=NOW, enabled=True, flags=KEEP)
+    def step(flags=KEEP):
+        return part.compact(ids, out_level=1, bottommost=1, now=NOW, enabled=True, flags=flags)
 
     for _ in range(args.warmup):
         res = step()
@@ -504,8 +600,9 @@ def main():
     w0 = time.perf_counter()
     with torch.cuda.stream(stream):
         ev0.record(stream)
-        for _ in range(args.steps):
-            res = step()
+        for i in range(args.steps):
+            # --dump-outputs: the last step installs its merged run so that it can be read back; the device work is the same
+            res = step(1 if args.dump_outputs and i == args.steps - 1 else KEEP)
             merge_ms.append(res.merge_kernel_ms)
             plan_ms.append(res.device_ms - res.merge_kernel_ms)
             walk_ms.append(res.walk_ms)
@@ -522,6 +619,10 @@ def main():
     max_ms = float(t.item())
     ms_per_step = max_ms / args.steps
     value = world * in_bytes / (ms_per_step / 1e3) / 1e9
+    if args.dump_outputs:
+        if rank == 0:
+            dump_compaction(args.dump_outputs, res, pgs.decode_blocks(part.download(res.new_run_id)))
+        part.drop(res.new_run_id)  # the read legs below see the same 4 runs as without the dump
 
     # ---- end to end through the C ABI from host buffers ------------------------------------------
     e2e = None
@@ -545,7 +646,7 @@ def main():
         barrier()
         split.update(upload=0.0, compact=0.0, drop=0.0)
         e0 = time.perf_counter()
-        n_e2e = max(1, min(args.steps, 3))
+        n_e2e = args.steps
         for _ in range(n_e2e):
             e2e_step()
         barrier()
@@ -594,11 +695,10 @@ def main():
         garena_cap = args.n_get * (VAL + 8)
         garena_buf = pinned_alloc(garena_cap, np.uint8)
         gres_buf = (pgs.GetResult * args.n_get)()
-        reps = max(3, args.steps)
         # gets
         part.get_batch(gkeys, goff, NOW, arena_cap=garena_cap, arena=garena_buf, results=gres_buf)
         g_ms, g_wall, found, probes = [], [], 0, 0
-        for _ in range(reps):
+        for _ in range(args.steps):
             barrier()
             t0 = time.perf_counter()
             st, gres, garena, gused = part.get_batch(gkeys, goff, NOW, arena_cap=garena_cap, arena=garena_buf, results=gres_buf)
@@ -611,7 +711,7 @@ def main():
         sb = part.prefix_scan_batch(hashkeys, max_records=80, arena_stride=24576, alloc=pinned_alloc)  # request structs marshalled once
         assert sb.run(NOW) == 0
         s_ms, s_wall = [], []
-        for _ in range(reps):
+        for _ in range(args.steps):
             barrier()
             t0 = time.perf_counter()
             st = sb.run(NOW)  # host request structs in, packed records out (host buffers)
@@ -619,6 +719,8 @@ def main():
             s_ms.append(eng.last_kernel_ms)
             assert st == 0, st
         sres, abase, kbase = sb.results, sb.abase, sb.kbase
+        if args.dump_outputs and rank == 0:
+            dump_reads(args.dump_outputs, gres, garena, sb)
         returned = int(kbase[-1])
         iterated = int(sum(sres[i].iter_count for i in range(args.n_scan)))
         scan_bytes = int(abase[-1])
@@ -701,7 +803,7 @@ def main():
     cpu, parity = None, None
     if rank == 0 and world == 1 and not args.skip_cpu:
         threads = os.cpu_count() or 1
-        gbs, secs, st = cpu_compaction(cpu_block_runs(runs), threads)
+        gbs, secs, st = cpu_compaction(cpu_block_runs(runs), threads)[:3]
         cpu = {"value": gbs, "unit": "GB/s", "cores": threads, "kind": "port",
                "what": "oracle-CPU block-level compaction (a restatement of the reference's RocksDB path, not RocksDB)",
                "sample": f"{RUNS} runs x {args.records_per_run} records ({st.in_bytes / 1e9:.2f} GB merged): the full workload, {secs:.2f} s"}
